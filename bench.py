@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the scan-matching hot path (BASELINE.json: correspondences/s per linearize()).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload): BASELINE.json configs[1] -- an IntegratedVGICPFactor with a 1,000,000-point source cloud
@@ -30,11 +30,13 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # the tree may be read-only: nothing is cached next to the sources
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -102,6 +104,17 @@ def make_poses(rank: int, count: int):
 
     rng = np.random.default_rng(1000 + rank)
     return np.stack([syn.random_pose(rng, POSE_ROT, POSE_TRANS) for _ in range(count)])
+
+
+def dump_records(out_dir, loop: str, records):
+    """Linearized records of a timed loop's last step ([F x >= 122] float64, b2_linearized layout) ->
+    out_dir/<loop>_<field>.npy, one float64 array per field with the factor as leading axis."""
+    from gtsam_points_b200 import capi
+
+    fields = [capi.unpack_linearized(r) for r in np.atleast_2d(np.asarray(records, dtype=np.float64))]
+    os.makedirs(out_dir, exist_ok=True)
+    for k in fields[0]:
+        np.save(os.path.join(out_dir, f"{loop}_{k}.npy"), np.array([f[k] for f in fields], dtype=np.float64))
 
 
 class ClockSampler:
@@ -209,9 +222,9 @@ def time_cpu(tp, tc, sp, sc, poses, warmup: int, steps: int):
     times = []
     for i in range(steps):
         t0 = time.perf_counter()
-        f.linearize_raw(poses[(warmup + i) % len(poses)])
+        last = f.linearize_raw(poses[(warmup + i) % len(poses)])
         times.append(time.perf_counter() - t0)
-    return times, threads
+    return times, threads, last
 
 
 def cpu_value(times) -> float:
@@ -222,10 +235,11 @@ def cpu_value(times) -> float:
 def time_cpu_native(steps: int, warmup: int):
     """Same oracle compiled with -march=native ON THIS HOST (the reference's BUILD_WITH_MARCH_NATIVE option, off by default):
     run in a child process because the library handle is process-global.  Returns correspondences/s or None."""
-    env = dict(os.environ, B2_ORACLE_NATIVE="1")
     try:
-        out = subprocess.run([sys.executable, os.path.abspath(__file__), "--impl", "reference", "--steps", str(steps), "--warmup", str(warmup), "--no-native"],
-                             env=env, capture_output=True, text=True, timeout=600, preexec_fn=lambda: os.sched_setaffinity(0, AFFINITY))
+        with tempfile.TemporaryDirectory(prefix="b2_oracle_native_") as tmp:
+            env = dict(os.environ, B2_ORACLE_NATIVE=tmp)
+            out = subprocess.run([sys.executable, os.path.abspath(__file__), "--impl", "reference", "--steps", str(steps), "--warmup", str(warmup), "--no-native"],
+                                 env=env, capture_output=True, text=True, timeout=600, preexec_fn=lambda: os.sched_setaffinity(0, AFFINITY))
         return float(json.loads(out.stdout.strip().splitlines()[-1])["value"])
     except Exception:
         return None
@@ -251,13 +265,15 @@ def run_reference(args):
     if rank != 0:
         return  # the CPU arm runs on rank 0 only
     tp, tc, sp, sc = make_inputs(0)
-    steps = max(args.steps, 10)  # median of >= 10 calls
+    steps = args.steps
     poses = make_poses(0, steps + args.warmup)
-    native = os.environ.get("B2_ORACLE_NATIVE") == "1"
+    native = bool(os.environ.get("B2_ORACLE_NATIVE"))
     # the -march=native child runs FIRST: afterwards this process's own OpenMP team exists and (OMP_WAIT_POLICY=active) spins
     # on the cores between parallel regions, which would steal them from the child
     native_value = time_cpu_native(steps, args.warmup) if (not native and not args.no_native) else None
-    times, threads = time_cpu(tp, tc, sp, sc, poses, args.warmup, steps)
+    times, threads, last = time_cpu(tp, tc, sp, sc, poses, args.warmup, steps)
+    if args.dump_outputs:
+        dump_records(args.dump_outputs, "linearize", last)  # same workload and last pose as the GPU arm's "linearize" loop
     value = cpu_value(times)
     sample = (f"median of {steps} linearize() calls of the full 1M-pt workload after {args.warmup} warm-up, one pinned OpenMP thread per physical core"
               + (", -march=native build" if native else ", reference default flags (-O3, no -march=native)"))
@@ -453,6 +469,7 @@ def run_gpu(args):
             t0 = time.perf_counter()
             out = e2e_step(poses_c[W + i], poses_p[W + i])
             e2e_s += time.perf_counter() - t0
+        e2e_rec = np.array(out, copy=True)
         barrier()
         clocks = sampler.stop() if rank == 0 else None
         e2e_ms = max_over_ranks(e2e_s * 1e3)
@@ -460,7 +477,7 @@ def run_gpu(args):
         # ================= sub-record: STRONG scaling -- the same 1M-point factor split over the ranks (SURVEY 8e(2)) =================
         # every rank holds the whole target map and a contiguous 1/N slice of rank 0's source cloud; the N partial records are
         # exchanged like any other records and summed (H, b and the error are sums over points)
-        strong = None
+        strong = strong_rec = None
         if world > 1 and not args.no_extra:
             tp0, tc0, sp0, sc0 = make_inputs(0)
             vm0 = g.GaussianVoxelMapGPU(RESOLUTION, ctx)
@@ -475,6 +492,7 @@ def run_gpu(args):
                 total["rec"] = ss.linearize_device(pose).sum(0)  # the factor's H, b, error = sum of the ranks' partial records
 
             ms_total, strong_ms = time_steps(strong_step, poses0, W, K, ss.device_barrier)
+            strong_rec = total["rec"].cpu().numpy()
             strong = {"workload": "ONE 1M-pt VGICP factor, source points split over the ranks, partial H/b records summed", "scaling": "strong",
                       "ms_per_step": ms_total / K, "step_ms_min_median_max": [float(strong_ms.min()), float(np.median(strong_ms)), float(strong_ms.max())], "value": N_SOURCE * K / (ms_total * 1e-3), "unit": UNIT, "inliers": int(total["rec"][121].item())}
             del ss, part, vm0
@@ -544,10 +562,18 @@ def run_gpu(args):
                       "oracle_inliers": int(ref[121]), "max_rel_err_H_b_error": rel}
             assert corr_equal and int(h_chk[0, 121]) == int(ref[121]) and rel < 1e-9, parity
 
+        if args.dump_outputs:
+            dump_records(args.dump_outputs, "linearize", rec)
+            dump_records(args.dump_outputs, "linearize_host", e2e_rec)
+            if strong_rec is not None:
+                dump_records(args.dump_outputs, "strong_scaling", strong_rec)
+            if cfg4 is not None:
+                dump_records(args.dump_outputs, "cfg4", rec4)
+
         cpu_baseline = None
         if world == 1 and not args.no_cpu_baseline:
             cs, cw = 10, 2
-            times, threads = time_cpu(tp, tc, sp, sc, poses, cw, cs)
+            times, threads, _ = time_cpu(tp, tc, sp, sc, poses, cw, cs)
             cpu_baseline = {
                 "value": cpu_value(times),
                 "unit": UNIT,
@@ -614,14 +640,17 @@ def run_gpu(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed linearize() calls of every measured loop")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the sub-records (strong-scaling split, cfg4 share): headline numbers only")
     ap.add_argument("--no-native", action="store_true", help="reference arm: skip the secondary -march=native measurement")
     ap.add_argument("--no-flush", action="store_true", help="diagnostic only: keep L2 warm between steps (NOT a valid bench number)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the H, b, error and inlier count that the last timed step of each timed loop computed to DIR/<loop>_<field>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     # Thread pinning is for the process that times the CPU oracle: the reference arm, or the single-process CUDA arm (cpu_baseline).

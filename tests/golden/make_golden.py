@@ -1,14 +1,16 @@
-"""Generates tests/golden/kitti07_pair.npz from the reference's own test data (run in the authoring container only).
+"""Generates tests/golden/kitti07_pair.npz from the reference's own test data.
 
-Inputs : /root/reference/data/kitti_07_dump/{graph.txt, 000000/points.bin, 000001/points.bin}  -- the submaps the reference's
+usage  : python tests/golden/make_golden.py <reference checkout>/data/kitti_07_dump
+Inputs : {graph.txt, 000000/points.bin, 000001/points.bin} of that directory -- the submaps the reference's
          src/test/test_matching_cost_factors.cpp:62-78 loads (packed float32 xyz; poses `tx ty tz qx qy qz qw`).
 Steps  : every 2nd point is kept (fixture size); covariances follow src/gtsam_points/features/covariance_estimation.cpp:18-77
          (k = 10 nearest neighbours incl. the point itself, cov = (sum p p^T - mean sum p^T) / k, eigenvalues replaced by
-         (1e-3, 1, 1) in ascending-eigenvalue order), computed here with brute-force numpy;
+         (1e-3, 1, 1) in ascending-eigenvalue order), computed by golden_util.estimate_covariances (the oracle) -- they are
+         not stored, the tests recompute them from the points the same way;
          noisy relative pose = ground truth composed with a fixed tangent perturbation;
          outputs = the CPU oracle's VGICP (1.0 m voxels, as in the reference test :84-90) and GICP linearize() / error() /
          correspondences with num_threads = 1 (deterministic summation order).
-The GPU box has no /root/reference: tests read only the .npz.
+Tests read only the .npz.
 """
 import os
 import sys
@@ -20,10 +22,9 @@ ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
+import golden_util  # noqa: E402
 import oracle_lib as orc  # noqa: E402
 from gtsam_points_b200 import synthetic as syn  # noqa: E402
-
-DATA = "/root/reference/data/kitti_07_dump"
 
 
 def quat_pose(v):
@@ -43,35 +44,17 @@ def quat_pose(v):
     return T
 
 
-def estimate_covariances(pts, k=10, eig=(1e-3, 1.0, 1.0), chunk=1024):
-    n = len(pts)
-    covs = np.zeros((n, 3, 3))
-    for s in range(0, n, chunk):
-        q = pts[s : s + chunk]
-        d = ((q[:, None, :] - pts[None, :, :]) ** 2).sum(-1)
-        idx = np.argpartition(d, k, axis=1)[:, :k]
-        nb = pts[idx]  # chunk x k x 3
-        sum_p = nb.sum(1)
-        sum_c = np.einsum("nki,nkj->nij", nb, nb)
-        mean = sum_p / k
-        c = (sum_c - mean[:, :, None] * sum_p[:, None, :]) / k
-        c = 0.5 * (c + c.transpose(0, 2, 1))
-        w, v = np.linalg.eigh(c)  # ascending eigenvalues, like SelfAdjointEigenSolver::computeDirect
-        covs[s : s + chunk] = np.einsum("nij,j,nkj->nik", v, np.array(eig), v)
-    return 0.5 * (covs + covs.transpose(0, 2, 1))
-
-
-def main():
+def main(data):
     poses = {}
-    for line in open(os.path.join(DATA, "graph.txt")):
+    for line in open(os.path.join(data, "graph.txt")):
         tok = line.split()
         poses[int(tok[0][1:])] = quat_pose([float(x) for x in tok[1:8]])
     clouds = []
     for i in (0, 1):
-        p = np.fromfile(os.path.join(DATA, f"{i:06d}", "points.bin"), dtype=np.float32).reshape(-1, 3)[::2]
+        p = np.fromfile(os.path.join(data, f"{i:06d}", "points.bin"), dtype=np.float32).reshape(-1, 3)[::2]
         clouds.append(np.ascontiguousarray(p))
     pts = [c.astype(np.float64) for c in clouds]
-    covs = [estimate_covariances(p) for p in pts]
+    covs = [golden_util.estimate_covariances(p) for p in pts]
 
     T_target, T_source_gt = poses[0], poses[1]
     xi = np.array([0.03, -0.02, 0.025, 0.08, -0.06, 0.04])  # fixed tangent noise (the reference test draws U(-0.1, 0.1))
@@ -84,8 +67,6 @@ def main():
     out = dict(
         target_points=clouds[0],
         source_points=clouds[1],
-        target_covs=np.stack([covs[0][:, 0, 0], covs[0][:, 0, 1], covs[0][:, 0, 2], covs[0][:, 1, 1], covs[0][:, 1, 2], covs[0][:, 2, 2]], 1),
-        source_covs=np.stack([covs[1][:, 0, 0], covs[1][:, 0, 1], covs[1][:, 0, 2], covs[1][:, 1, 1], covs[1][:, 1, 2], covs[1][:, 2, 2]], 1),
         T_target=T_target,
         T_source_gt=T_source_gt,
         T_source=T_source,
@@ -113,4 +94,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

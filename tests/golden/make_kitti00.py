@@ -1,12 +1,13 @@
-"""Generates tests/golden/kitti00_pair.npz from the reference's data/kitti_00 (run in the authoring container only).
+"""Generates tests/golden/kitti00_pair.npz from the reference's data/kitti_00.
 
-Inputs : /root/reference/data/kitti_00/000000.bin, 000001.bin -- packed float32 xyz (util/read_points.hpp:30-45), the two
+usage  : python tests/golden/make_kitti00.py <reference checkout>/data/kitti_00
+Inputs : 000000.bin, 000001.bin of that directory -- packed float32 xyz (util/read_points.hpp:30-45), the two
          consecutive KITTI-00 scans the reference ships (BASELINE.json configs[4], SURVEY.md 8d cfg5).
-Steps  : every 2nd point is kept (fixture size; 62,334 + 62,303 points); the test estimates covariances the way
+Steps  : every 3rd point is kept (fixture size; 41,556 + 41,535 points); the test estimates covariances the way
          src/gtsam_points/features/covariance_estimation.cpp:18-77 does (k = 10, EIG regularisation) with the oracle, builds a
          0.5 m GaussianVoxelMap from frame 0 and runs the frame-to-map LM of tests/mini_lm.py from identity.
 Outputs: the points (float32, as in the files) and the ORACLE-driven LM pose track + final pose as golden values.
-The GPU box has no /root/reference: tests read only the .npz.
+Tests read only the .npz.
 """
 import os
 import sys
@@ -21,7 +22,6 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import mini_lm  # noqa: E402
 import oracle_lib as orc  # noqa: E402
 
-DATA = "/root/reference/data/kitti_00"
 RESOLUTION = 0.5
 
 
@@ -36,8 +36,8 @@ def oracle_track(p0, p1, threads=4):
     return vm, values[0], np.stack(track), hist
 
 
-def main():
-    frames = [np.fromfile(os.path.join(DATA, f"{i:06d}.bin"), dtype=np.float32).reshape(-1, 3)[::2].copy() for i in (0, 1)]
+def main(data):
+    frames = [np.fromfile(os.path.join(data, f"{i:06d}.bin"), dtype=np.float32).reshape(-1, 3)[::3].copy() for i in (0, 1)]
     p0, p1 = (f.astype(np.float64) for f in frames)
     vm, T, track, hist = oracle_track(p0, p1)
     out = os.path.join(HERE, "kitti00_pair.npz")
@@ -48,4 +48,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

@@ -17,10 +17,13 @@ LINEARIZED_DOUBLES = 122
 
 
 def build(force=False):
-    if os.environ.get("B2_ORACLE_NATIVE") == "1":
-        # secondary CPU number of bench.py: the same code with -march=native, ALWAYS rebuilt on the host that runs it
-        subprocess.check_call(["make", "-B", "-C", ORACLE_DIR, "liboracle_native.so"], stdout=subprocess.DEVNULL)
-        return os.path.join(ORACLE_DIR, "liboracle_native.so")
+    native_dir = os.environ.get("B2_ORACLE_NATIVE")
+    if native_dir:
+        # secondary CPU number of bench.py: the same code with -march=native, ALWAYS rebuilt on the host that runs it, into the
+        # directory B2_ORACLE_NATIVE names (bench.py runs from a tree that may be read-only)
+        so = os.path.join(os.path.abspath(native_dir), "liboracle_native.so")
+        subprocess.check_call(["make", "-B", "-C", ORACLE_DIR, f"NATIVE_OUT={so}", so], stdout=subprocess.DEVNULL)
+        return so
     so = os.path.join(ORACLE_DIR, "liboracle.so")
     src = [os.path.join(ORACLE_DIR, f) for f in ("oracle.cpp", "oracle.h", "Makefile")]
     if force or not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in src):

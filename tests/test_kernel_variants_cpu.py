@@ -26,6 +26,7 @@ def test_alternative_kernel_forms_compile_and_the_tma_form_contains_tma(tmp_path
         results = list(ex.map(lambda i: _compile(i, str(tmp_path / f"factors_impl{i}.o")), impls))
     for impl, r in zip(impls, results):
         assert r.returncode == 0, f"B2_VGICP_IMPL={impl} no longer compiles:\n{r.stderr[-2000:]}"
-    sass = subprocess.run(["cuobjdump", "-sass", str(tmp_path / "factors_impl2.o")], capture_output=True, text=True).stdout
+    cuobjdump = os.path.join(os.path.dirname(b2build.NVCC), "cuobjdump")  # the toolkit's bin/ need not be on PATH
+    sass = subprocess.run([cuobjdump, "-sass", str(tmp_path / "factors_impl2.o")], capture_output=True, text=True).stdout
     for mnemonic in ("UBLKCP", "SYNCS.ARRIVE.TRANS64", "SYNCS.PHASECHK.TRANS64.TRYWAIT", "LDGSTS", "USETMAXREG"):
         assert mnemonic in sass, f"{mnemonic} missing from the TMA-staged kernel's SASS"

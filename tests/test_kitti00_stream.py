@@ -45,7 +45,7 @@ def test_oracle_reproduces_the_golden_pose_track(data):
     # a plausible KITTI ego-motion: ~0.68 m forward, < 0.01 rad
     rot, trans = mini_lm.pose_error(T, np.eye(4))
     assert 0.5 < trans < 0.9 and rot < 0.01
-    # hit rate at identity (SURVEY.md 8d: 77 % of the full scan at 0.5 m; the half-density fixture sees a sparser map)
+    # hit rate at identity (SURVEY.md 8d: 77 % of the full scan at 0.5 m; the third-density fixture sees a sparser map)
     assert 0.4 < vm.overlap(orc.Cloud(data["p1"], data["c1"]), np.eye(4)) < 0.95
 
 
